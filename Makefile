@@ -27,30 +27,16 @@ $(BUILD)/%.o: %.cpp
 oracle:
 	$(MAKE) -C oracle
 
-# The reference's own benchmark drivers, compiled UNCHANGED from where they lie under $(REF)
-# against mpr_b200/inc + mpr_b200/shim and linked with libmprb.so (drop-in check).
-REF ?= /root/reference
-DRIVERS := render_2d_table render_3d_table print_tape_table tape_building_time circle tape_shortening \
-           render_effects render_2d render_3d render_2d_heatmap render_3d_heatmap dump_tape
-# render_2d / render_3d also write an out_cpu.png through libfive's CPU renderer; its stand-in
-# (mpr_b200/shim/src/heightmap_render.cpp) is linked into the drivers only, never into libmprb.so.
-# brute.cu carries a kernel of its own, so it goes through nvcc.
-drivers: mpr_b200/libmprb.so
-	@mkdir -p $(BUILD)/drivers && \
-	  $(CXX) -O2 -std=c++17 -Impr_b200/inc -Impr_b200/shim -c mpr_b200/shim/src/heightmap_render.cpp \
-	    -o $(BUILD)/drivers/heightmap_render.o && \
-	  $(CXX) -O2 -std=c++17 -Impr_b200/inc -Impr_b200/shim tests/cpp/heightmap_check.cpp \
-	    $(BUILD)/drivers/heightmap_render.o -Lmpr_b200 -lmprb -pthread \
-	    -Wl,-rpath,'$$ORIGIN/../../mpr_b200' -o $(BUILD)/drivers/heightmap_check
-	@if [ -d $(REF)/benchmark ]; then \
-	  for d in $(DRIVERS); do \
-	  $(CXX) -O2 -std=c++17 -Impr_b200/inc -Impr_b200/shim -I$(REF)/benchmark \
-	    $(REF)/benchmark/$$d.cpp $(REF)/benchmark/stats.cpp $(BUILD)/drivers/heightmap_render.o -Lmpr_b200 -lmprb \
-	    -pthread -Wl,-rpath,'$$ORIGIN/../../mpr_b200' -o $(BUILD)/drivers/$$d || exit 1; done && \
-	  $(NVCC) -O2 -std=c++17 $(ARCH) -Impr_b200/inc -Impr_b200/shim -I$(REF)/benchmark \
-	    $(REF)/benchmark/brute.cu $(REF)/benchmark/stats.cpp -Lmpr_b200 -lmprb \
-	    -Xlinker -rpath -Xlinker '$$ORIGIN/../../mpr_b200' -o $(BUILD)/drivers/brute; \
-	else echo "reference sources not present; keeping prebuilt $(BUILD)/drivers (if any)"; fi
+# tests/cpp/heightmap_check: the CPU renderer stand-in the reference's drivers link (oracle/Makefile builds
+# those), checked on the drivers' default shape.  mpr_b200/shim/src/heightmap_render.cpp is linked into test
+# programs and drivers only, never into libmprb.so.
+drivers: $(BUILD)/drivers/heightmap_check
+
+$(BUILD)/drivers/heightmap_check: tests/cpp/heightmap_check.cpp mpr_b200/shim/src/heightmap_render.cpp mpr_b200/libmprb.so
+	@mkdir -p $(dir $@)
+	$(CXX) -O2 -std=c++17 -Impr_b200/inc -Impr_b200/shim tests/cpp/heightmap_check.cpp \
+	    mpr_b200/shim/src/heightmap_render.cpp -Lmpr_b200 -lmprb -pthread \
+	    -Wl,-rpath,'$$ORIGIN/../../mpr_b200' -o $@
 
 clean:
 	rm -rf $(BUILD) mpr_b200/libmprb.so

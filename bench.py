@@ -13,6 +13,7 @@ final device synchronisation.
   python bench.py [--gpus N] [--steps K] [--warmup W]          this repository's CUDA path
   python bench.py --impl reference ...                         the UNMODIFIED reference CUDA
                                                                renderer (oracle/_ref), same workload
+  python bench.py ... --dump-outputs DIR                       also write what the last timed frame computed
 Both arms also time the CPU restatement (oracle/) on the host cores as `cpu_baseline`.
 Under torchrun (N > 1) every rank renders a band of 64-px tile rows and the bands are
 exchanged with one NCCL all-gather per frame.
@@ -167,6 +168,30 @@ def golden_digest(case: str):
 def digest(a: np.ndarray) -> str:
     import hashlib
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()[:32]
+
+
+DUMP_BUDGET = 60 << 20      # bytes of array data --dump-outputs writes, all files together (< 64 MB with headers)
+
+
+def dump_outputs(out_dir: str, jobs, holder: str):
+    """--dump-outputs: the image (and in 3D the normals) that job[holder] - a context of either arm - holds
+    for every workload, as <out_dir>/<model>_<dim>d_<size>_<image|normals>.npy in float64, which holds the
+    int32 depth and 0 / 1 images and the packed uint32 normals exactly.  An array larger than its equal share
+    of DUMP_BUDGET is written as a fixed sample instead: the elements at the flat indices
+    np.random.default_rng(0) draws (without replacement, increasing), the same in every run."""
+    arrays = {}
+    for j in jobs:
+        case = f"{j['model']}_{j['dim']}d_{j['size']}"
+        arrays[f"{case}_image"] = np.array(j[holder].image())
+        if j["dim"] == 3:
+            arrays[f"{case}_normals"] = np.array(j[holder].normals())
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    share = DUMP_BUDGET // 8 // len(arrays)
+    for name, a in arrays.items():
+        if a.size > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(out / f"{name}.npy", a.astype(np.float64))
 
 
 # Launch order inside one frame (mpr_b200/csrc/api.cu: render()).
@@ -374,6 +399,8 @@ def run_mine(args, workloads):
     dev = np.array([step(frame_device) for _ in range(args.steps)])      # [K, n_jobs] device ms
     barrier()
     t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs and rank == 0:     # the last timed frame (after the exchange when N > 1)
+        dump_outputs(args.dump_outputs, jobs, "ctx")
     launches = sum(j["ctx"].stats().n_launches for j in jobs)
     dev_digest = {}
     if world > 1 and rank == 0:     # what the NCCL exchange left on rank 0's device after the last timed frame
@@ -573,6 +600,8 @@ def run_reference(args, workloads):
     clocks = ClockSampler(0)
     clocks.start()
     dev = np.array([step(frame) for _ in range(args.steps)])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, jobs, "ref")
     for _ in range(min(args.warmup, 3)):
         step(frame_e2e)
     e2e = np.array([step(frame_e2e) for _ in range(args.steps)])
@@ -666,6 +695,9 @@ def main():
                     help="comma list of <model>_<2d|3d>_<size>, or 'sweep' = the reference's table sizes "
                          "(prospero 2D 256..4096, bear 3D 256..1536)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write each workload's image (and 3D normals) of the last timed "
+                         "frame as DIR/<model>_<dim>d_<size>_<image|normals>.npy, float64, < 64 MB in all")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     # NCCL takes its debug level from the environment it was loaded under: with several ranks, make sure

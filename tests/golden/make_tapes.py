@@ -6,7 +6,9 @@ contract starts at the packed tape, SURVEY.md section 8c).  They are produced by
 this repository's own .frep reader + tape packer (libmprb: mprb_tape_from_frep),
 with libfive's load-time simplification rules switched on.
 
-Run here (needs /root/reference; no GPU):  python tests/golden/make_tapes.py
+The .frep models under tests/golden/frep are the reference's benchmark/files, unchanged.
+
+No GPU needed:  python tests/golden/make_tapes.py
 """
 import hashlib
 import json
@@ -19,7 +21,7 @@ ROOT = Path(__file__).resolve().parents[2]
 sys.path.insert(0, str(ROOT))
 from mpr_b200 import capi  # noqa: E402
 
-SRC = Path("/root/reference/benchmark/files")
+SRC = Path(__file__).resolve().parent / "frep"
 OUT = Path(__file__).resolve().parent / "tapes"
 MODELS = ["prospero", "involute_gear_2d", "involute_gear_3d", "architecture", "bear", "hello_world"]
 

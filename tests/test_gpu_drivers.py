@@ -1,6 +1,6 @@
 """Drop-in check on the GPU box: the reference's own benchmark drivers, compiled unchanged
-against mpr_b200/inc and linked with libmprb.so (`make drivers`, prebuilt binaries travel in
-build/drivers), run and produce their tables / images."""
+against mpr_b200/inc and linked with libmprb.so (`make -C oracle drivers`, which keeps what it built
+in oracle/_ref/drivers where the reference sources are absent), run and produce their tables / images."""
 import re
 import subprocess
 
@@ -10,7 +10,7 @@ import pytest
 from conftest import ROOT
 
 pytestmark = pytest.mark.gpu
-DRV = ROOT / "build" / "drivers"
+DRV = ROOT / "oracle" / "_ref" / "drivers"
 
 
 def run(name, cwd, *args, timeout=300):

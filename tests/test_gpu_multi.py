@@ -62,7 +62,7 @@ def test_multi_gpu_context_equals_single_gpu_frame(model, dim, size):
 
 @need2
 def test_reference_table_driver_runs_on_two_gpus(tmp_path):
-    exe = ROOT / "build" / "drivers" / "render_3d_table"
+    exe = ROOT / "oracle" / "_ref" / "drivers" / "render_3d_table"
     if not exe.exists():
         pytest.skip("drivers not built")
     env = dict(os.environ, MPRB_GPUS="2")

@@ -1,9 +1,11 @@
 """GPU parity tests (B200 box): libmprb through its C ABI against
   (1) fixtures minted from the unmodified reference build (tests/golden/ref),
-  (2) the reference build itself when oracle/_ref/libmpr_ref.so travelled with the snapshot,
+  (2) what the reference build computed for post-effects, brute-force frames and work meters
+      (tests/golden/ref_variants, minted by tools/mint_ref_variants.py),
   (3) the CPU restatement,
 and size-independent properties at the BASELINE sizes.  Integer / byte results: bit exact."""
 import ctypes as C
+import json
 
 import numpy as np
 import pytest
@@ -17,6 +19,11 @@ pytestmark = pytest.mark.gpu
 SUBTAPES = 6400000
 CASES = golden_cases()
 SMALL = [c for c in CASES if c[5] is not None]
+VARIANTS = ROOT / "tests" / "golden" / "ref_variants"
+
+
+def ref_variant(key):
+    return json.loads((VARIANTS / "records.json").read_text())[key]
 
 
 def render(model, dim, size, **kw):
@@ -43,18 +50,17 @@ def test_matches_reference_fixture(case):
     ctx.close()
 
 
-@pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("model,dim,size", [("prospero", 2, 512), ("involute_gear_2d", 2, 1024),
                                             ("architecture", 3, 512), ("bear", 3, 512),
                                             ("involute_gear_3d", 3, 512)])
 def test_matches_live_reference_build(model, dim, size):
-    cells = load_tape(model)
-    ref = oracle.RefGpu(size)
-    (ref.render2D if dim == 2 else ref.render3D)(cells)
-    ref_fp = parity.fingerprint(ref, dim)
-    ref.close()
+    """Every field of the fingerprint equals the reference build's frame (its digests, recorded in
+    tests/golden/ref by tools/gpu_check.py)."""
+    want = json.loads((ROOT / "tests" / "golden" / "ref" / f"{model}_{dim}d_{size}.json").read_text())
     ctx, tape = render(model, dim, size)
-    assert not parity.compare(ref_fp, parity.fingerprint(ctx, dim))
+    got = parity.summarize(parity.fingerprint(ctx, dim))
+    assert set(got) == set(want)
+    assert not parity.compare_summary(want, got)
     ctx.close()
 
 
@@ -347,38 +353,30 @@ def test_small_levels_evaluated_clause_parallel_give_the_reference_frame(name, w
     ctx.close()
 
 
-@pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("model,size", [("bear", 256), ("architecture", 512), ("bear", 1024)])
 def test_effects_match_reference_build(model, size):
     """mpr::Effects::drawSSAO / drawShaded against the reference's own src/effects.cu, compiled unmodified
-    into oracle/_ref (with the Eigen stand-in of oracle/shim for its small-vector algebra), on the same
-    frame and the same sample sets: bit for bit, both result buffers."""
-    cells = load_tape(model)
-    ref = oracle.RefGpu(size)
-    ref.render3D(cells)
-    rfx = oracle.RefEffects()
-    kernel, rvecs = rfx.samples()
+    (with the Eigen stand-in of oracle/shim for its small-vector algebra), on the same frame and the same
+    sample sets: bit for bit, both result buffers (their digests and the sample sets the reference drew
+    are recorded in tests/golden/ref_variants)."""
+    want = ref_variant(f"effects/{model}_{size}")
+    samples = np.load(VARIANTS / f"effects_{model}_{size}.npz")
     ctx, tape = render(model, 3, size)
-    assert np.array_equal(ctx.image(), ref.image()) and np.array_equal(ctx.normals(), ref.normals())
-    fx = capi.Effects(kernel, rvecs)
+    assert parity.digest(ctx.image()) == want["image"] and parity.digest(ctx.normals()) == want["normals"]
+    fx = capi.Effects(samples["kernel"], samples["rvecs"])
     for shaded in (False, True):
-        want_image, want_tmp = rfx.draw(ref, shaded=shaded)
+        effect = "shaded" if shaded else "ssao"
         (fx.drawShaded if shaded else fx.drawSSAO)(ctx)
-        got_image, got_tmp = fx.image().copy(), fx.tmp().copy()
-        for name, got, want in (("image", got_image, want_image), ("tmp", got_tmp, want_tmp)):
-            bad = int((got != want).sum())
-            assert bad == 0, (model, size, "shaded" if shaded else "ssao", name, bad,
-                              np.argwhere(got != want)[:4].tolist())
+        got = {"image": parity.digest(fx.image()), "tmp": parity.digest(fx.tmp())}
+        assert got == want[effect], (model, size, effect)
     fx.close()
-    rfx.close()
     ctx.close()
-    ref.close()
 
 
 @pytest.mark.parametrize("model,size", [("hello_world", 256), ("prospero", 512)])
 def test_brute_force_frame(model, size):
     """Context::render2D_brute (context.cu:1461-1508): same image as the subdivided frame, as the
-    CPU restatement and - when it travelled - the reference build produce it."""
+    CPU restatement and the reference build produce it."""
     cells = load_tape(model)
     ctx, tape = render(model, 2, size)
     fancy = ctx.image().copy()
@@ -390,11 +388,7 @@ def test_brute_force_frame(model, size):
     o.render2D_brute(cells)
     assert np.array_equal(got, o.image())
     o.close()
-    if oracle.ref_available():
-        r = oracle.RefGpu(size)
-        r.render2D_brute(cells)
-        assert np.array_equal(got, r.image())
-        r.close()
+    assert parity.digest(got) == ref_variant(f"brute/{model}_{size}")["image"]
     ctx.render2D(tape)                       # the context is still good for ordinary frames
     assert np.array_equal(ctx.image(), fancy)
     ctx.close()
@@ -414,11 +408,8 @@ def test_work_meter_2d_is_exact(model, size):
     want, units = o.render2D_heatmap(cells)
     assert np.array_equal(heat, want)
     o.close()
-    if oracle.ref_available():
-        r = oracle.RefGpu(size)
-        ref = r.render2D_heatmap(cells)
-        np.testing.assert_allclose(heat, ref, rtol=2e-5, atol=0)
-        r.close()
+    ref = np.load(VARIANTS / f"heatmap2d_{model}_{size}.npz")["heat"]
+    np.testing.assert_allclose(heat, ref, rtol=2e-5, atol=0)
     ctx.close()
 
 
@@ -442,9 +433,5 @@ def test_work_meter_3d(model, size):
     want, _ = o.render3D_heatmap(cells)
     assert 1 / 1.6 < float(heat.sum()) / float(want.sum()) < 1.6
     o.close()
-    if oracle.ref_available():
-        r = oracle.RefGpu(size)
-        ref = r.render3D_heatmap(cells)
-        assert 1 / 1.6 < float(heat.sum()) / float(ref.sum()) < 1.6
-        r.close()
+    assert 1 / 1.6 < float(heat.sum()) / ref_variant(f"heatmap3d/{model}_{size}")["sum"] < 1.6
     ctx.close()

@@ -4,7 +4,6 @@ import ctypes as C
 import hashlib
 import json
 import re
-from pathlib import Path
 
 import numpy as np
 import pytest
@@ -12,7 +11,7 @@ import pytest
 from conftest import GOLDEN, MODELS, ROOT, load_tape
 from mpr_b200 import capi
 
-REF_FILES = Path("/root/reference/benchmark/files")
+FREP_FILES = GOLDEN / "frep"          # the reference's benchmark models (benchmark/files/*.frep), as shipped
 
 
 def test_library_exports_every_declared_symbol():
@@ -43,10 +42,9 @@ SURVEY = {"prospero": (6056, 85, 2354), "involute_gear_2d": (1660, 67, 374), "in
           "architecture": (1296, 93, 488), "bear": (544, 23, 27), "hello_world": (328, 27, 97)}
 
 
-@pytest.mark.skipif(not REF_FILES.exists(), reason="reference fixtures not present on this box")
 @pytest.mark.parametrize("model", MODELS)
 def test_frep_reader_and_packer_reproduce_committed_tapes(model):
-    data = (REF_FILES / f"{model}.frep").read_bytes()
+    data = (FREP_FILES / f"{model}.frep").read_bytes()
     cells = capi.tape_from_frep(data, simplify=True)
     assert np.array_equal(cells, load_tape(model))
     clauses, slots, choices = SURVEY[model]
@@ -196,9 +194,9 @@ def test_dump_tape_reproduces_the_kernel_libfive_generated_for_brute_cu():
     Tree stand-in must print the same statements in the same order - a known answer for operator
     overloads, hash-consing, commutative rebalancing and orderedDfs together."""
     import subprocess
-    exe = ROOT / "build" / "drivers" / "dump_tape"
+    exe = ROOT / "oracle" / "_ref" / "drivers" / "dump_tape"
     if not exe.exists():
-        pytest.skip("build/drivers/dump_tape not built (needs the reference sources at build time)")
+        pytest.skip("oracle/_ref/drivers/dump_tape not built (needs the reference sources at build time)")
     out = subprocess.run([str(exe)], capture_output=True, text=True, timeout=60).stdout
     names = {}
     body = []

@@ -52,6 +52,9 @@ CASES = [
     ("prospero", 2, 512),
     ("prospero", 2, 3072),
     ("bear", 3, 512),
+    # the frames tests/test_gpu_parity.py::test_matches_live_reference_build checks
+    ("architecture", 3, 512),
+    ("involute_gear_3d", 3, 512),
 ]
 
 SUBTAPES = 6400000   # the reference arm is built with -DBIG_SERVER

@@ -8,5 +8,5 @@ python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127
 tail -c 600 $O/bench_n$N.json; grep -c "nranks" $O/bench_n$N.err
 done
 timeout 600 python -m pytest tests/test_gpu_multi.py -x -q > $O/pytest_multi.log 2>&1; tail -3 $O/pytest_multi.log
-for G in 1 8; do MPRB_GPUS=$G timeout 300 ./build/drivers/render_3d_table 2>&1 | tail -8 > $O/render_3d_table_g$G.log; cat $O/render_3d_table_g$G.log; done
+for G in 1 8; do MPRB_GPUS=$G timeout 300 ./oracle/_ref/drivers/render_3d_table 2>&1 | tail -8 > $O/render_3d_table_g$G.log; cat $O/render_3d_table_g$G.log; done
 python tools/multi_gpu_times.py bear:3:1024 prospero:2:4096 > $O/multi_gpu_times.log 2>&1; cat $O/multi_gpu_times.log
